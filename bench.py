@@ -5,6 +5,8 @@
     python bench.py --impl reference --gpus N --steps K ...  # reference arm: the CPU restatement of the
                                                              # reference's own algorithm on the host cores
   N > 1 is launched by `python -m torch.distributed.run --nproc-per-node N ...` (one rank per GPU).
+  --dump-outputs DIR writes what the headline's last timed step computed (see dump_outputs); the inputs are seeded, so two
+  builds run with the same arguments can be compared output for output.
 
 A "step" = one pass of the hot path over one batch: BASELINE.json configs[1], secp256k1 variable-base
 scalar multiplication of 2^20 (scalar, point) pairs per GPU (weak scaling: each rank owns its own 2^20 pairs,
@@ -218,6 +220,30 @@ class ClockSampler:
         return {"sm_mhz": float(np.median(load)), "sm_max_mhz": max(mx), "power_w_max": max(power), "samples": len(sm), "reasons": sorted(reasons)}
 
 
+DUMP_ROWS = 1 << 17   # per-element outputs larger than this are dumped as a fixed sample of rows (<= 34 MB in all)
+DUMP_SEED = 0xB2000D00
+
+
+def dump_outputs(out_dir, op, n, out_xy, out_inf):
+    """Write what one step of the timed path returned to its caller as float32 .npy files (byte values 0..255, exact):
+    mul / mulgen -> xy [rows, 64] (big-endian x || y) + inf [rows]; lincomb -> the one sum point; schnorr -> valid [rows].
+    Batches above DUMP_ROWS are sampled at fixed, seeded row indices (index.npy), so two builds can be compared row for row."""
+    os.makedirs(out_dir, exist_ok=True)
+    if op == "lincomb":
+        arrays = {"xy": out_xy.reshape(1, 64), "inf": out_inf[:1]}
+    else:
+        idx = np.arange(n) if n <= DUMP_ROWS else np.sort(np.random.default_rng(DUMP_SEED).choice(n, DUMP_ROWS, replace=False))
+        arrays = {"index": idx}
+        if op == "schnorr":
+            arrays["valid"] = out_xy[idx]
+        else:
+            arrays["xy"] = out_xy.reshape(n, 64)[idx]
+            arrays["inf"] = out_inf[idx]
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a, dtype=np.float32))
+    return sorted(arrays)
+
+
 def dist_setup(n_gpus):
     import torch
 
@@ -317,9 +343,10 @@ class Bench:
         return float(t.item())
 
 
-def measure(B, workload, steps, warmup, sample_clocks):
+def measure(B, workload, steps, warmup, sample_clocks, dump_dir=None):
     """One BASELINE config on this job's ranks: device-resident rate (`value`), end-to-end rate through the host-buffer ABI,
-    bit-exact comparison of EVERY output with the CPU restatement, roofline.  Returns the record on rank 0, None elsewhere."""
+    bit-exact comparison of EVERY output with the CPU restatement, roofline.  Returns the record on rank 0, None elsewhere.
+    dump_dir: rank 0 writes the device path's outputs of the last timed step there (dump_outputs)."""
     import torch
 
     import ecref
@@ -431,6 +458,7 @@ def measure(B, workload, steps, warmup, sample_clocks):
     ms_per_step = ms_total / steps
     value = world * n * steps / (ms_total * 1e-3)
     dev_xy, dev_inf = oxy.cpu().numpy().copy(), oinf.cpu().numpy().copy()
+    dumped = dump_outputs(dump_dir, op, n, dev_xy, dev_inf) if (dump_dir and rank == 0) else None
     exch = None
     if exchange:
         # the same call without the exchange step (every rank reduces and normalises its own terms): what the NCCL
@@ -558,6 +586,8 @@ def measure(B, workload, steps, warmup, sample_clocks):
     }
     if clocks is not None:
         rec["clocks"] = clocks
+    if dumped is not None:
+        rec["dumped_outputs"] = {"dir": os.path.abspath(dump_dir), "arrays": dumped, "rank": 0}
     if exch is not None:
         rec["exchange"] = exch
     return rec
@@ -1149,20 +1179,20 @@ def measure_ecdsa_recover(B, steps):
 def run_ours(args):
     B = Bench(args)
     world, rank = B.world, B.rank
-    line = measure(B, args.workload, args.steps, args.warmup, sample_clocks=True)
+    line = measure(B, args.workload, args.steps, args.warmup, sample_clocks=True, dump_dir=args.dump_outputs)
     configs = {}
     if args.configs == "all" and args.workload == "k256_varbase":
-        sub_steps = max(3, min(args.steps, args.sub_steps))
+        sub_steps = min(args.steps, args.sub_steps)
         if rank == 0:
             configs["1_k256_plumbing_cpu"] = config1_plumbing(B)
         for key, wl in (("3_p256_varbase", "p256_varbase"), ("4_k256_fixedbase", "k256_fixedbase"), ("5_k256_lincomb", "k256_lincomb")):
             configs[key] = measure(B, wl, sub_steps, 3, sample_clocks=False)
-        configs["6_p384_varbase"] = measure_p384(B, max(3, sub_steps // 2))
-        configs["7_more_curves"] = measure_more_curves(B, 3)
-        configs["8_consttime_cost"] = measure_consttime_cost(B, 5)
-        configs["9_hash_to_curve"] = measure_hash_to_curve(B, 5)
+        configs["6_p384_varbase"] = measure_p384(B, sub_steps)
+        configs["7_more_curves"] = measure_more_curves(B, sub_steps)
+        configs["8_consttime_cost"] = measure_consttime_cost(B, sub_steps)
+        configs["9_hash_to_curve"] = measure_hash_to_curve(B, sub_steps)
         configs["10_k256_schnorr_verify"] = measure(B, "k256_schnorr_verify", sub_steps, 3, sample_clocks=False)
-        configs["11_k256_ecdsa_recover"] = measure_ecdsa_recover(B, 5)
+        configs["11_k256_ecdsa_recover"] = measure_ecdsa_recover(B, sub_steps)
         if world > 1:
             configs["strong_scaling"] = strong_scaling(B)
             barrier_sync(world)
@@ -1239,16 +1269,20 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=40)
+    ap.add_argument("--steps", type=int, default=40, help="timed steps of the headline workload (and, up to --sub-steps, of every other record)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="k256_varbase", choices=sorted(WORKLOADS))
     ap.add_argument("--log2-batch", type=int, default=0, help="override the per-GPU batch (development only)")
     ap.add_argument("--configs", default="all", choices=["all", "none"],
                     help="all: the headline line also carries a `configs` object with BASELINE.json configs 1, 3, 4, 5 (+ strong scaling at N > 1)")
-    ap.add_argument("--sub-steps", type=int, default=10, help="timed steps of the non-headline configs")
+    ap.add_argument("--sub-steps", type=int, default=10, help="cap on the timed steps of the non-headline configs: they run min(--steps, --sub-steps)")
     ap.add_argument("--strong-log2", type=int, default=23, help="log2 of the strong-scaling batch (N > 1)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the headline's outputs of its last timed step to DIR/<name>.npy (float32; sampled rows above 2^17)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
     if args.impl == "reference":
         run_reference(args)
     else:

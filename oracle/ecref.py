@@ -23,16 +23,29 @@ def _host_tag():
     return hashlib.sha1(flags.encode()).hexdigest()
 
 
-def build(force=False):
-    tagf = LIB + ".host"
+def _make(lib_path, srcs, force=False):
+    """(Re)build one oracle library with make when it is missing, older than its sources or built for another CPU."""
+    tagf = lib_path + ".host"
     tag = _host_tag()
-    stale = (not os.path.exists(LIB) or os.path.getmtime(LIB) < os.path.getmtime(os.path.join(_HERE, "ecref.c"))
+    srcs = [os.path.join(_HERE, s) for s in srcs]
+    stale = (not os.path.exists(lib_path) or os.path.getmtime(lib_path) < max(os.path.getmtime(s) for s in srcs)
              or not os.path.exists(tagf) or open(tagf).read().strip() != tag)
     if force or stale:
-        subprocess.check_call(["make", "-C", _HERE, "-B", "libecref.so"], stdout=subprocess.DEVNULL)
+        subprocess.check_call(["make", "-C", _HERE, "-B", os.path.basename(lib_path)], stdout=subprocess.DEVNULL)
         with open(tagf, "w") as f:
             f.write(tag)
-    return LIB
+    return lib_path
+
+
+def build(force=False):
+    return _make(LIB, ["ecref.c"], force)
+
+
+def build_all(force=False):
+    """Every oracle library with its CPU tag, so that later loads on this machine write nothing into the tree."""
+    build(force)
+    _make(LIB384, ["ecref_p384.c"], force)
+    _make(LIBP, ["ecref_prime.c", "ecref_prime_impl.inc"], force)
 
 
 def lib():
@@ -67,14 +80,7 @@ def lib384():
     """oracle/ecref_p384.c — the P-384 restatement (48-byte records)"""
     global _lib384
     if _lib384 is None:
-        tagf = LIB384 + ".host"
-        tag = _host_tag()
-        src = os.path.join(_HERE, "ecref_p384.c")
-        if (not os.path.exists(LIB384) or os.path.getmtime(LIB384) < os.path.getmtime(src) or not os.path.exists(tagf)
-                or open(tagf).read().strip() != tag):
-            subprocess.check_call(["make", "-C", _HERE, "-B", "libecref384.so"], stdout=subprocess.DEVNULL)
-            with open(tagf, "w") as f:
-                f.write(tag)
+        _make(LIB384, ["ecref_p384.c"])
         _lib384 = ctypes.CDLL(LIB384)
         _lib384.ecref384_init()
         vp, sz = ctypes.c_void_p, ctypes.c_size_t
@@ -96,14 +102,7 @@ def libp():
     """oracle/ecref_prime.c — the generic primeorder / Montgomery-field restatement (sm2, brainpool, bign, P-224, P-192)"""
     global _libp
     if _libp is None:
-        tagf = LIBP + ".host"
-        tag = _host_tag()
-        srcs = [os.path.join(_HERE, "ecref_prime.c"), os.path.join(_HERE, "ecref_prime_impl.inc")]
-        if (not os.path.exists(LIBP) or os.path.getmtime(LIBP) < max(os.path.getmtime(f) for f in srcs) or not os.path.exists(tagf)
-                or open(tagf).read().strip() != tag):
-            subprocess.check_call(["make", "-C", _HERE, "-B", "libecrefp.so"], stdout=subprocess.DEVNULL)
-            with open(tagf, "w") as f:
-                f.write(tag)
+        _make(LIBP, ["ecref_prime.c", "ecref_prime_impl.inc"])
         _libp = ctypes.CDLL(LIBP)
         _libp.ecrefp_init()
         vp, sz = ctypes.c_void_p, ctypes.c_size_t
