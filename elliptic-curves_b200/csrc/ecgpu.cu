@@ -29,6 +29,9 @@
 #if ECG_TU == 0
 #include "ecg_microbench.cuh"
 #endif
+#if ECG_TU == 1  // SM2 public-key encryption (sm2 only)
+#include "ecg_sm2pke.cuh"
+#endif
 #include "ecg_msm.cuh"
 
 #define ECG_CURVE_COUNT 12
@@ -1095,6 +1098,12 @@ __attribute__((visibility("hidden"))) ecg_status ecg_tu4_ecg_lincomb_partial(ecg
 __attribute__((visibility("hidden"))) ecg_status ecg_tu4_ecg_point_sum(ecg_ctx* ctx, ecg_curve curve, size_t m, const uint8_t* xyz, uint8_t* out_xy, uint8_t* out_inf);
 __attribute__((visibility("hidden"))) ecg_status ecg_tu4_ecg_lincomb(ecg_ctx* ctx, ecg_curve curve, size_t n, const uint8_t* k, const uint8_t* P_xy, const uint8_t* P_inf, uint8_t* out_xy, uint8_t* out_inf);
 __attribute__((visibility("hidden"))) ecg_status ecg_tu1_ecg_sm2dsa_verify_batch(ecg_ctx* ctx, size_t n, const uint8_t* e32, const uint8_t* sig64, const uint8_t* Q_xy, uint8_t* valid);
+__attribute__((visibility("hidden"))) ecg_status ecg_tu1_ecg_sm2pke_encrypt_batch(ecg_ctx* ctx, size_t n, const uint8_t* msgs, const uint64_t* offsets,
+                                                                                const uint8_t* k32, const uint8_t* Pb_xy, int mode, int compressed,
+                                                                                uint8_t* out, uint8_t* status);
+__attribute__((visibility("hidden"))) ecg_status ecg_tu1_ecg_sm2pke_decrypt_batch(ecg_ctx* ctx, size_t n, const uint8_t* cts, const uint64_t* offsets,
+                                                                                const uint8_t* d32, int mode, uint8_t* out, uint64_t* pt_len,
+                                                                                uint8_t* valid);
 __attribute__((visibility("hidden"))) ecg_status ecg_tu1_ecg_mul_gen_add_batch(ecg_ctx* ctx, ecg_curve curve, size_t n, const uint8_t* a, const uint8_t* b, const uint8_t* P_xy, const uint8_t* P_inf, uint8_t* out_xy, uint8_t* out_inf);
 __attribute__((visibility("hidden"))) ecg_status ecg_tu1_ecg_ecdsa_verify_batch(ecg_ctx* ctx, ecg_curve curve, size_t n, const uint8_t* z32, const uint8_t* sig64, const uint8_t* Q_xy, int low_s_only, uint8_t* valid);
 __attribute__((visibility("hidden"))) ecg_status ecg_tu2_ecg_mul_gen_add_batch(ecg_ctx* ctx, ecg_curve curve, size_t n, const uint8_t* a, const uint8_t* b, const uint8_t* P_xy, const uint8_t* P_inf, uint8_t* out_xy, uint8_t* out_inf);
@@ -1305,6 +1314,161 @@ ECG_API(ecg_sm2dsa_verify_batch)(ecg_ctx* ctx, size_t n, const uint8_t* e32, con
   op.out = valid;
   op.ostride = 1;
   return run_batch(ctx, op, n);
+#else
+  return ECG_EINVAL;
+#endif
+}
+
+#if ECG_TU == 1
+// ---- SM2 public-key encryption (ecg_sm2pke.cuh): one pass on device 0, lane 0 ---------------------------------------
+// front end -> variable-base [k]Pb / [d]C1 -> affine (x2, y2) -> (encryption: [k]G -> affine C1) -> KDF / C3 / layout
+static ecg_status sm2pke_run(ecg_ctx* ctx, bool enc, size_t n, const uint8_t* data, const uint64_t* offsets, const uint8_t* key32,
+                             const uint8_t* pb_xy, int mode, int compressed, uint8_t* out, uint8_t* verdict, uint64_t* pt_len) {
+  DevState& d = ctx->devs[0];
+  Lane& L = d.lane[0];
+  CU_TRY(ctx, cudaSetDevice(d.dev));
+  const bool ct = (ctx->flags & ECG_FLAG_CONSTTIME) != 0;
+  if (enc && !ct) ST_TRY(ensure_fb_table(ctx, d, ECG_SM2));
+  ST_TRY(begin_lane(ctx, L));
+  const size_t ovh = enc ? 32 + (compressed ? 33 : 65) : 0;
+  const uint8_t *ddata = data, *dkey = key32, *dpb = pb_xy;
+  const uint64_t* doffs = offsets;
+  uint8_t *dout = out, *dverdict = verdict;
+  uint64_t* dlen = pt_len;
+  uint64_t base = 0;
+  size_t out_bytes = 0;
+  if (!ctx->devptr()) {
+    base = offsets[0];
+    const size_t total = (size_t)(offsets[n] - base);
+    out_bytes = total + n * ovh;
+    ST_TRY(ensure(ctx, L, B_P, total + 16));
+    ST_TRY(ensure(ctx, L, B_K, (n + 1) * 8));
+    ST_TRY(ensure(ctx, L, B_A, n * 32));
+    if (total) CU_TRY(ctx, cudaMemcpyAsync(L.buf[B_P], data + base, total, cudaMemcpyHostToDevice, L.s()));
+    CU_TRY(ctx, cudaMemcpyAsync(L.buf[B_K], offsets, (n + 1) * 8, cudaMemcpyHostToDevice, L.s()));
+    CU_TRY(ctx, cudaMemcpyAsync(L.buf[B_A], key32, n * 32, cudaMemcpyHostToDevice, L.s()));
+    ddata = (const uint8_t*)L.buf[B_P];
+    doffs = (const uint64_t*)L.buf[B_K];
+    dkey = (const uint8_t*)L.buf[B_A];
+    if (enc) {
+      ST_TRY(ensure(ctx, L, B_X, n * 64));
+      CU_TRY(ctx, cudaMemcpyAsync(L.buf[B_X], pb_xy, n * 64, cudaMemcpyHostToDevice, L.s()));
+      dpb = (const uint8_t*)L.buf[B_X];
+    }
+    ST_TRY(ensure(ctx, L, B_OUT, out_bytes + 16));
+    ST_TRY(ensure(ctx, L, B_OINF, n));
+    dout = (uint8_t*)L.buf[B_OUT];
+    dverdict = (uint8_t*)L.buf[B_OINF];
+    if (!enc) {
+      ST_TRY(ensure(ctx, L, B_AUX, n * 8));
+      dlen = (uint64_t*)L.buf[B_AUX];
+    }
+  }
+  ST_TRY(ensure(ctx, L, B_V1, n * 64));
+  ST_TRY(ensure(ctx, L, B_V2, n * 32));
+  ST_TRY(ensure(ctx, L, B_V4, n));
+  ST_TRY(ensure(ctx, L, B_V5, n * 64));
+  ST_TRY(ensure(ctx, L, B_V6, n));
+  ST_TRY(ensure(ctx, L, B_JAC, n * jbytes(ECG_SM2)));
+  uint8_t *vp = (uint8_t*)L.buf[B_V1], *vk = (uint8_t*)L.buf[B_V2], *vok = (uint8_t*)L.buf[B_V4];
+  uint8_t *vxy = (uint8_t*)L.buf[B_V5], *vinf = (uint8_t*)L.buf[B_V6];
+  if (enc)
+    sm2pke_enc_prep_kernel<CurveSm2><<<grid_for(n, 128), 128, 0, L.s()>>>(doffs, n, dkey, dpb, vk, vp, vok);
+  else
+    sm2pke_dec_prep_kernel<CurveSm2><<<grid_for(n, 128), 128, 0, L.s()>>>(ddata, doffs, base, n, dkey, vk, vp, vok);
+  LAUNCHED(ctx);
+  DevPtrs dp;
+  dp.k = vk;
+  dp.p = vp;
+  ST_TRY(launch_varbase(ctx, d, L, ECG_SM2, n, dp, (uint32_t*)L.buf[B_JAC], L.status, 0));
+  ST_TRY(launch_norm(ctx, d, L, ECG_SM2, n, (uint32_t*)L.buf[B_JAC], vxy, vinf));
+  const uint8_t* c1xy = nullptr;
+  if (enc) {  // C1 = [k]G: the fixed-base table, or under ECG_FLAG_CONSTTIME the variable-base routine with P = G
+    ST_TRY(ensure(ctx, L, B_JAC2, n * jbytes(ECG_SM2)));
+    ST_TRY(ensure(ctx, L, B_V3, n * 64));
+    ST_TRY(ensure(ctx, L, B_INF, n));
+    uint32_t* jac2 = (uint32_t*)L.buf[B_JAC2];
+    if (ct) {
+      DevPtrs g;
+      g.k = vk;
+      ST_TRY(launch_varbase(ctx, d, L, ECG_SM2, n, g, jac2, L.status, 0));
+    } else {
+      DOM_BEGIN(ctx, L);
+      fixedbase_kernel<CurveSm2><<<grid_for(n, 128), 128, 0, L.s()>>>(vk, n, d.fb_table[ECG_SM2], jac2, L.status, 0);
+      LAUNCHED(ctx);
+      DOM_END(ctx, L);
+    }
+    ST_TRY(launch_norm(ctx, d, L, ECG_SM2, n, jac2, (uint8_t*)L.buf[B_V3], (uint8_t*)L.buf[B_INF]));
+    c1xy = (const uint8_t*)L.buf[B_V3];
+  }
+  if (enc)
+    sm2pke_kdf_kernel<true><<<grid_for(n, 128), 128, 0, L.s()>>>(ddata, doffs, base, n, mode, compressed, vxy, c1xy, vok, dout, dverdict, nullptr);
+  else
+    sm2pke_kdf_kernel<false><<<grid_for(n, 128), 128, 0, L.s()>>>(ddata, doffs, base, n, mode, 0, vxy, nullptr, vok, dout, dverdict, dlen);
+  LAUNCHED(ctx);
+  if (!ctx->devptr()) {
+    if (out_bytes) CU_TRY(ctx, cudaMemcpyAsync(out, dout, out_bytes, cudaMemcpyDeviceToHost, L.s()));
+    CU_TRY(ctx, cudaMemcpyAsync(verdict, dverdict, n, cudaMemcpyDeviceToHost, L.s()));
+    if (!enc) CU_TRY(ctx, cudaMemcpyAsync(pt_len, dlen, n * 8, cudaMemcpyDeviceToHost, L.s()));
+  }
+  return ECG_OK;
+}
+
+static ecg_status sm2pke_entry(ecg_ctx* ctx, bool enc, size_t n, const uint8_t* data, const uint64_t* offsets, const uint8_t* key32,
+                               const uint8_t* pb_xy, int mode, int compressed, uint8_t* out, uint8_t* verdict, uint64_t* pt_len) {
+  const char* who = enc ? "ecg_sm2pke_encrypt_batch" : "ecg_sm2pke_decrypt_batch";
+  if (n == 0) return ECG_OK;
+  if (!offsets || !key32 || !out || !verdict || (enc && !pb_xy) || (!enc && !pt_len) || n > ((size_t)1 << 31)) {
+    ctx->err = std::string(who) + ": null pointer";
+    return ECG_EINVAL;
+  }
+  if (mode != 0 && mode != 1) {
+    ctx->err = std::string(who) + ": mode must be 0 (C1C3C2) or 1 (C1C2C3)";
+    return ECG_EINVAL;
+  }
+  if (ctx->devptr()) {
+    if (!data || (reinterpret_cast<uintptr_t>(offsets) & 7) || (reinterpret_cast<uintptr_t>(key32) & 3) ||
+        (reinterpret_cast<uintptr_t>(pb_xy) & 3) || (reinterpret_cast<uintptr_t>(pt_len) & 7)) {
+      ctx->err = std::string(who) + ": null device pointer, or offsets / pt_len not 8-byte aligned, or keys not 4-byte aligned";
+      return ECG_EINVAL;
+    }
+  } else {
+    for (size_t i = 0; i < n; i++)
+      if (offsets[i + 1] < offsets[i]) {
+        ctx->err = std::string(who) + ": offsets must be non-decreasing";
+        return ECG_EINVAL;
+      }
+    if (!data && offsets[n] != offsets[0]) {
+      ctx->err = std::string(who) + ": null data buffer";
+      return ECG_EINVAL;
+    }
+  }
+  ecg_status st = sm2pke_run(ctx, enc, n, data, offsets, key32, pb_xy, mode, compressed, out, verdict, pt_len);
+  if (st != ECG_OK) return fail(ctx, st);
+  st = finish(ctx);
+  return st == ECG_OK ? st : fail(ctx, st);
+}
+#endif  // ECG_TU == 1
+
+// SM2 public-key encryption: TU 1 holds sm2; the public entries (TU 0) forward there
+ECG_API(ecg_sm2pke_encrypt_batch)(ecg_ctx* ctx, size_t n, const uint8_t* msgs, const uint64_t* offsets, const uint8_t* k32,
+                                  const uint8_t* Pb_xy, int mode, int compressed, uint8_t* out, uint8_t* status) {
+  if (!ctx) return ECG_EINVAL;
+#if ECG_TU == 0
+  return ecg_tu1_ecg_sm2pke_encrypt_batch(ctx, n, msgs, offsets, k32, Pb_xy, mode, compressed, out, status);
+#elif ECG_TU == 1
+  return sm2pke_entry(ctx, true, n, msgs, offsets, k32, Pb_xy, mode, compressed, out, status, nullptr);
+#else
+  return ECG_EINVAL;
+#endif
+}
+ECG_API(ecg_sm2pke_decrypt_batch)(ecg_ctx* ctx, size_t n, const uint8_t* cts, const uint64_t* offsets, const uint8_t* d32, int mode,
+                                  uint8_t* out, uint64_t* pt_len, uint8_t* valid) {
+  if (!ctx) return ECG_EINVAL;
+#if ECG_TU == 0
+  return ecg_tu1_ecg_sm2pke_decrypt_batch(ctx, n, cts, offsets, d32, mode, out, pt_len, valid);
+#elif ECG_TU == 1
+  return sm2pke_entry(ctx, false, n, cts, offsets, d32, nullptr, mode, 0, out, valid, pt_len);
 #else
   return ECG_EINVAL;
 #endif

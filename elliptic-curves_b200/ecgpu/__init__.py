@@ -9,6 +9,8 @@ bench.py.  It mirrors the reference's names for the hot path:
     Engine.mul_by_generator_and_mul_add(...)   MulByGeneratorVartime::..._and_mul_add    (mul.rs:303-310)
     Engine.batch_normalize(curve, XYZ)         BatchNormalize::batch_normalize           (projective.rs:345-391)
     Engine.field_op(curve, op, a, b)           FieldElement add/sub/neg/mul/square/invert
+    Engine.sm2pke_encrypt / sm2pke_decrypt     sm2 EncryptingKey::encrypt / DecryptingKey::decrypt over a batch
+                                               (`*_vartime` on a ctx without ECG_FLAG_CONSTTIME)
 
 Buffers are numpy uint8 arrays (host mode) or raw device pointers (device mode, ECG_FLAG_DEVICE_PTRS).
 There is NO CPU fallback: if libecgpu.so is missing, or no CUDA device is present, construction raises.
@@ -53,7 +55,10 @@ EXPORTS = [
     "ecg_schnorr_verify_batch", "ecg_ecdsa_verify_batch", "ecg_decompress_batch",
     "ecg_batch_normalize_hom", "ecg_mul_batch_x", "ecg_field_sqrt_batch",
     "ecg_hash_to_curve_batch", "ecg_hash_to_scalar_batch", "ecg_sm2dsa_verify_batch", "ecg_ecdsa_recover_batch",
+    "ecg_sm2pke_encrypt_batch", "ecg_sm2pke_decrypt_batch",
 ]
+# SM2 public-key encryption ciphertext layouts (sm2/src/pke.rs Mode; C1C3C2 is the reference's default)
+SM2PKE_MODES = {"c1c3c2": 0, "c1c2c3": 1, 0: 0, 1: 1}
 
 
 class EcgError(RuntimeError):
@@ -138,6 +143,10 @@ def load_library(path: Optional[str] = None) -> ctypes.CDLL:
     lib.ecg_hash_to_curve_batch.restype = ctypes.c_int
     lib.ecg_hash_to_scalar_batch.argtypes = [vp, ctypes.c_int, sz, u8p, u8p, u8p, sz, u8p]
     lib.ecg_hash_to_scalar_batch.restype = ctypes.c_int
+    lib.ecg_sm2pke_encrypt_batch.argtypes = [vp, sz, u8p, u8p, u8p, u8p, ctypes.c_int, ctypes.c_int, u8p, u8p]
+    lib.ecg_sm2pke_encrypt_batch.restype = ctypes.c_int
+    lib.ecg_sm2pke_decrypt_batch.argtypes = [vp, sz, u8p, u8p, u8p, ctypes.c_int, u8p, u8p, u8p]
+    lib.ecg_sm2pke_decrypt_batch.restype = ctypes.c_int
     lib.ecg_version.argtypes = []
     lib.ecg_version.restype = ctypes.c_char_p
     if path is None:
@@ -178,6 +187,7 @@ class Engine:
         arr = (ctypes.c_int * len(devs))(*devs)
         self._ctx = ctypes.c_void_p(0)
         self.device_ptrs = device_ptrs
+        self.consttime = consttime
         flags = (FLAG_DEVICE_PTRS if device_ptrs else 0) | (FLAG_ZEROIZE if zeroize else 0) | (FLAG_CONSTTIME if consttime else 0)
         rc = self.lib.ecg_ctx_create(arr, len(devs), flags, ctypes.byref(self._ctx))
         if rc != ECG_OK:
@@ -421,6 +431,103 @@ class Engine:
         valid = np.zeros(n, np.uint8)
         self._check(self.lib.ecg_sm2dsa_verify_batch(self._ctx, n, _ptr(e32), _ptr(sig64), _ptr(Q_xy), _ptr(valid)))
         return valid
+
+    # ---- SM2 public-key encryption (ecg_sm2pke_{encrypt,decrypt}_batch; sm2/src/pke/{encrypting,decrypting}.rs) ----
+    # Without ECG_FLAG_CONSTTIME the scalar multiplications by k and d run the variable-time kernels, so, as with
+    # diffie_hellman_vartime, the methods of a default ctx carry the `_vartime` suffix; an Engine(consttime=True) serves
+    # the plain names.  Engine(zeroize=True) scrubs d, k, the staged messages and plaintexts and (x2, y2) after each call.
+    def _sm2pke_ct(self, name):
+        if not self.consttime:
+            raise ValueError(f"{name}: this Engine runs the variable-time kernels; create it with consttime=True or call {name}_vartime")
+
+    @staticmethod
+    def _broadcast(a, rec: int, n: int, name: str) -> np.ndarray:
+        """one record (broadcast to all n elements) or n records of `rec` bytes"""
+        a = np.ascontiguousarray(np.frombuffer(bytes(a), np.uint8) if isinstance(a, (bytes, bytearray)) else a, dtype=np.uint8).reshape(-1)
+        if a.size == rec:
+            return np.ascontiguousarray(np.broadcast_to(a, (n, rec))).reshape(-1) if n else np.zeros(rec, np.uint8)
+        return _u8(a, rec * n, name)
+
+    def sm2pke_encrypt_packed_vartime(self, data, offsets, k, Pb, mode="c1c3c2", compressed: bool = True):
+        """SM2 encryption of messages laid out as the C ABI takes them (`data` back to back, n + 1 uint64 `offsets`), with
+        the caller's ephemeral scalars k (n x 32 bytes) and the recipient key(s) Pb (64 bytes x || y, or n x 64)
+        -> (out, out_offsets, status): ciphertext i = out[out_offsets[i]:out_offsets[i + 1]] (zero bytes unless status[i]
+        = 1); status 0 = refused (k not in [1, n-1], Pb off the curve, empty message), 2 = all-zero KDF output: draw
+        another k (the reference's retry loop, encrypting.rs:184-209)."""
+        offs = np.ascontiguousarray(offsets, dtype=np.uint64)
+        n = offs.size - 1
+        data = np.ascontiguousarray(data, dtype=np.uint8).reshape(-1)
+        if n < 0 or int(offs[-1]) > data.size:
+            raise ValueError("offsets: n + 1 non-decreasing byte offsets into data")
+        if data.size == 0:
+            data = np.zeros(1, np.uint8)
+        k = _u8(k, 32 * n, "k")
+        Pb = self._broadcast(Pb, 64, n, "Pb")
+        ovh = 32 + (33 if compressed else 65)
+        out_offs = (offs - offs[0]) + np.arange(n + 1, dtype=np.uint64) * np.uint64(ovh) if n >= 0 else offs
+        out = np.zeros(max(int(out_offs[-1]), 1), np.uint8)
+        status = np.zeros(n, np.uint8)
+        self._check(self.lib.ecg_sm2pke_encrypt_batch(self._ctx, n, _ptr(data), _ptr(offs), _ptr(k), _ptr(Pb), SM2PKE_MODES[mode],
+                                                      1 if compressed else 0, _ptr(out), _ptr(status)))
+        return out[:int(out_offs[-1])], out_offs, status
+
+    def sm2pke_decrypt_packed_vartime(self, data, offsets, d, mode="c1c3c2"):
+        """SM2 decryption of packed ciphertexts (C1 in any SEC1 form the reference accepts) under the secret key(s) d
+        (32 bytes, or n x 32) -> (out, pt_len, valid): plaintext i = out[offsets[i] - offsets[0]:][:pt_len[i]]"""
+        offs = np.ascontiguousarray(offsets, dtype=np.uint64)
+        n = offs.size - 1
+        data = np.ascontiguousarray(data, dtype=np.uint8).reshape(-1)
+        if n < 0 or int(offs[-1]) > data.size:
+            raise ValueError("offsets: n + 1 non-decreasing byte offsets into data")
+        if data.size == 0:
+            data = np.zeros(1, np.uint8)
+        d = self._broadcast(d, 32, n, "d")
+        total = int(offs[-1] - offs[0]) if n > 0 else 0
+        out = np.zeros(max(total, 1), np.uint8)
+        pt_len = np.zeros(n, np.uint64)
+        valid = np.zeros(n, np.uint8)
+        self._check(self.lib.ecg_sm2pke_decrypt_batch(self._ctx, n, _ptr(data), _ptr(offs), _ptr(d), SM2PKE_MODES[mode], _ptr(out),
+                                                      _ptr(pt_len), _ptr(valid)))
+        return out[:total], pt_len, valid
+
+    def sm2pke_encrypt_vartime(self, msgs, k, Pb, mode="c1c3c2", compressed: bool = True):
+        """EncryptingKey::encrypt over a list of messages (sm2/src/pke/encrypting.rs:166-230, digest SM3) with the caller's k
+        -> (ciphertexts, status): ciphertext i is bytes where status[i] = 1, else None"""
+        data, offs = self._pack_messages(msgs)
+        out, oo, status = self.sm2pke_encrypt_packed_vartime(data, offs, k, Pb, mode, compressed)
+        return [out[int(oo[i]):int(oo[i + 1])].tobytes() if status[i] == 1 else None for i in range(len(msgs))], status
+
+    def sm2pke_decrypt_vartime(self, cts, d, mode="c1c3c2"):
+        """DecryptingKey::decrypt over a list of ciphertexts (sm2/src/pke/decrypting.rs:174-222) -> plaintext bytes, or None
+        where the reference returns Err"""
+        data, offs = self._pack_messages(cts)
+        out, pt_len, valid = self.sm2pke_decrypt_packed_vartime(data, offs, d, mode)
+        return [out[int(offs[i]):int(offs[i]) + int(pt_len[i])].tobytes() if valid[i] else None for i in range(len(cts))]
+
+    def sm2pke_encrypt(self, msgs, k, Pb, mode="c1c3c2", compressed: bool = True):
+        self._sm2pke_ct("sm2pke_encrypt")
+        return self.sm2pke_encrypt_vartime(msgs, k, Pb, mode, compressed)
+
+    def sm2pke_decrypt(self, cts, d, mode="c1c3c2"):
+        self._sm2pke_ct("sm2pke_decrypt")
+        return self.sm2pke_decrypt_vartime(cts, d, mode)
+
+    def sm2pke_encrypt_packed(self, data, offsets, k, Pb, mode="c1c3c2", compressed: bool = True):
+        self._sm2pke_ct("sm2pke_encrypt_packed")
+        return self.sm2pke_encrypt_packed_vartime(data, offsets, k, Pb, mode, compressed)
+
+    def sm2pke_decrypt_packed(self, data, offsets, d, mode="c1c3c2"):
+        self._sm2pke_ct("sm2pke_decrypt_packed")
+        return self.sm2pke_decrypt_packed_vartime(data, offsets, d, mode)
+
+    def sm2pke_encrypt_ptr(self, n, msgs, offsets, k32, Pb_xy, mode, compressed, out, status):
+        """device-pointer mode (device_ptrs=True): every argument an integer CUDA address"""
+        self._check(self.lib.ecg_sm2pke_encrypt_batch(self._ctx, n, _ptr(msgs), _ptr(offsets), _ptr(k32), _ptr(Pb_xy), SM2PKE_MODES[mode],
+                                                      1 if compressed else 0, _ptr(out), _ptr(status)))
+
+    def sm2pke_decrypt_ptr(self, n, cts, offsets, d32, mode, out, pt_len, valid):
+        self._check(self.lib.ecg_sm2pke_decrypt_batch(self._ctx, n, _ptr(cts), _ptr(offsets), _ptr(d32), SM2PKE_MODES[mode], _ptr(out),
+                                                      _ptr(pt_len), _ptr(valid)))
 
     def decompress_batch(self, curve, sec1_33):
         """AffinePoint::decompress over a batch of (1 + FB)-byte SEC1 compressed records -> (xy, inf, valid)"""

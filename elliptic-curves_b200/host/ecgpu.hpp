@@ -11,6 +11,7 @@
 //   Engine::batch_normalize(jacobian)                 <->  BatchNormalize::batch_normalize     (projective.rs:345-365)
 //   Engine::hash_to_curve / encode_to_curve / hash_to_scalar <-> GroupDigest::hash_from_bytes / encode_from_bytes,
 //                                                         hash2curve::hash_to_scalar (hash2curve/src/group_digest.rs:88-143)
+//   Engine::sm2pke_encrypt / sm2pke_decrypt          <->  sm2::pke::EncryptingKey::encrypt / DecryptingKey::decrypt
 // The typed surface below is for the 256-bit curves with big-endian records (secp256k1, P-256, sm2, brainpoolP256r1/t1);
 // the other curves of include/ecgpu.h (48 / 28 / 24-byte records, bign's little-endian records) are reached through the
 // C ABI directly or the Python mirror, which sizes its buffers per curve.
@@ -251,6 +252,49 @@ class Engine {
     std::vector<Scalar> r(n);
     check(ecg_hash_to_scalar_batch(ctx_, curve_, n, reinterpret_cast<const uint8_t*>(all.data()), offs.data(),
                                    reinterpret_cast<const uint8_t*>(dst.data()), dst.size(), reinterpret_cast<uint8_t*>(r.data())));
+    return r;
+  }
+
+  // SM2 public-key encryption, digest SM3 (Engine(ECG_SM2, ...) only; mode 0 = C1C3C2, 1 = C1C2C3).
+  // EncryptingKey::encrypt over a batch (sm2/src/pke/encrypting.rs:166-230) with the caller's ephemeral scalars k: one
+  // recipient key, one ciphertext per message; an empty vector where status != 1 (0 refused, 2: draw another k).
+  std::vector<std::vector<uint8_t>> sm2pke_encrypt(const AffinePoint& pb, const std::vector<Scalar>& k, const std::vector<std::string>& msgs,
+                                                   int mode = 0, bool compressed = true, std::vector<uint8_t>* status = nullptr) {
+    const size_t n = check_sizes(k.size(), msgs.size()), ovh = 32 + (compressed ? 33 : 65);
+    std::vector<uint64_t> offs(n + 1, 0);
+    std::string all;
+    for (size_t i = 0; i < n; i++) {
+      all += msgs[i];
+      offs[i + 1] = all.size();
+    }
+    pack(std::vector<AffinePoint>(n, pb));
+    std::vector<uint8_t> out(all.size() + n * ovh), st(n);
+    check(ecg_sm2pke_encrypt_batch(ctx_, n, reinterpret_cast<const uint8_t*>(all.data()), offs.data(), flat(k), xy_.data(), mode,
+                                   compressed ? 1 : 0, out.data(), st.data()));
+    std::vector<std::vector<uint8_t>> r(n);
+    for (size_t i = 0; i < n; i++)
+      if (st[i] == 1) r[i].assign(out.begin() + offs[i] + i * ovh, out.begin() + offs[i + 1] + (i + 1) * ovh);
+    if (status) *status = st;
+    return r;
+  }
+  // DecryptingKey::decrypt over a batch (sm2/src/pke/decrypting.rs:174-222): one secret key; valid[i] = 0 where the
+  // reference returns Err (its plaintext is then empty)
+  std::vector<std::vector<uint8_t>> sm2pke_decrypt(const Scalar& d, const std::vector<std::vector<uint8_t>>& cts, int mode = 0,
+                                                   std::vector<bool>* valid = nullptr) {
+    const size_t n = cts.size();
+    std::vector<uint64_t> offs(n + 1, 0), len(n);
+    std::vector<uint8_t> all;
+    for (size_t i = 0; i < n; i++) {
+      all.insert(all.end(), cts[i].begin(), cts[i].end());
+      offs[i + 1] = all.size();
+    }
+    std::vector<Scalar> ds(n, d);
+    std::vector<uint8_t> out(all.size()), ok(n);
+    check(ecg_sm2pke_decrypt_batch(ctx_, n, all.data(), offs.data(), flat(ds), mode, out.data(), len.data(), ok.data()));
+    std::vector<std::vector<uint8_t>> r(n);
+    for (size_t i = 0; i < n; i++)
+      if (ok[i]) r[i].assign(out.begin() + offs[i], out.begin() + offs[i] + len[i]);
+    if (valid) valid->assign(ok.begin(), ok.end());
     return r;
   }
 

@@ -54,8 +54,8 @@ typedef enum {
  * defines ECDSA for (all but sm2 and bign-curve256v1, whose signature schemes differ); hash to curve the four curves with
  * an RFC 9380 suite in the reference; SEC1 decompression every curve (one exponentiation by (p + 1) / 4 where p = 3 mod 4,
  * Tonelli-Shanks for P-224); the field square root every curve but P-224 (where the reference's root is the one its
- * external bignum crate's Tonelli-Shanks happens to return); BIP340 is secp256k1's alone and SM2DSA sm2's.  What a curve
- * does not serve answers ECG_EINVAL. */
+ * external bignum crate's Tonelli-Shanks happens to return); BIP340 is secp256k1's alone, SM2DSA and SM2 public-key
+ * encryption sm2's.  What a curve does not serve answers ECG_EINVAL. */
 typedef enum {
   ECG_SECP256K1 = 0,
   ECG_NISTP256 = 1,
@@ -91,7 +91,8 @@ typedef enum {
                                    memset per buffer and call */
 
 #define ECG_FLAG_CONSTTIME 4u   /* scalar-independent execution for the entries that take secret scalars — ecg_mul_batch[_x],
-                                   ecg_mul_gen_batch, ecg_lincomb[_partial] — the analogue of the reference's constant-time
+                                   ecg_mul_gen_batch, ecg_lincomb[_partial], the scalar multiplications of
+                                   ecg_sm2pke_{encrypt,decrypt}_batch — the analogue of the reference's constant-time
                                    `Mul` / `lincomb` (k256/src/arithmetic/mul.rs:112-163, LookupTable::select
                                    primeorder/src/tables/lookup.rs:43-65): window-table entries are fetched by a masked scan
                                    over all entries, the GLV sign folding is branch-free, k*G runs through the variable-base
@@ -195,6 +196,33 @@ ecg_status ecg_ecdsa_recover_batch(ecg_ctx* ctx, ecg_curve curve, size_t n, cons
  * verdict; its group step R = (s1 + H)*G + (s0 + 2^128)*Q is ecg_mul_gen_add_batch on ECG_BIGNP256. */
 ecg_status ecg_sm2dsa_verify_batch(ecg_ctx* ctx, size_t n, const uint8_t* e32, const uint8_t* sig64, const uint8_t* Q_xy,
                                    uint8_t* valid);
+
+/* SM2 public-key encryption (GB/T 32918.4; curve sm2 only, so no curve argument), digest SM3.  Records are variable-length
+ * and packed as for hash to curve: record i = data[offsets[i] .. offsets[i+1]), n + 1 non-decreasing uint64 offsets.  With
+ * ECG_FLAG_DEVICE_PTRS every data pointer is a device pointer (offsets and pt_len 8-byte aligned, k32 / d32 / Pb_xy
+ * 4-byte aligned) and the offsets are not checked on the host.  Both entries run on the ctx's first device.  A bad
+ * ciphertext, key or nonce is a per-record verdict, not an API error; ECG_EINVAL means a null pointer, decreasing
+ * offsets, an unknown mode or a misaligned device pointer.  mode 0 = C1C3C2 (the reference's default), 1 = C1C2C3.
+ *
+ * C_i = SM2-Enc(Pb_i, M_i; k_i).  k32: n*32 ephemeral scalars (the caller's randomness; the reference draws k inside,
+ * sm2/src/pke/encrypting.rs:186-188), Pb_xy: n*64 recipient keys.  compressed != 0: C1 = 02|03 || x (what
+ * EncryptingKey::encrypt emits, encrypting.rs:90), else 04 || x || y (OpenSSL / GM/T 0003 interoperability).
+ * Record i is written at out + (offsets[i] - offsets[0]) + i*ovh, ovh = 32 + (compressed ? 33 : 65), length len_i + ovh,
+ * laid out as Cipher::to_slice (sm2/src/pke.rs:181-213).  status[i]: 1 = ok; 0 = refused (k not in [1, n-1], Pb not
+ * on the curve, empty message), record zeroed; 2 = the KDF output was all zero, draw another k (the reference's retry
+ * loop, encrypting.rs:184-209), record zeroed.  Replaces EncryptingKey::encrypt / encrypt_digest::<_, Sm3>
+ * (encrypting.rs:166-230). */
+ecg_status ecg_sm2pke_encrypt_batch(ecg_ctx* ctx, size_t n, const uint8_t* msgs, const uint64_t* offsets, const uint8_t* k32,
+                                    const uint8_t* Pb_xy, int mode, int compressed, uint8_t* out, uint8_t* status);
+
+/* M_i = SM2-Dec(d_i, C_i).  Ciphertext i = cts[offsets[i] .. offsets[i+1]), C1 in any SEC1 form the reference accepts
+ * (02 / 03 compressed, 04 uncompressed, 05 compact; Cipher::from_slice, sm2/src/pke.rs:122-160).  d32: n*32 secret
+ * scalars, valid only in [1, n-1].  out has the size of cts: plaintext i at out + (offsets[i] - offsets[0]), pt_len[i]
+ * bytes; every other byte of record i's range is written as zero, as is the whole range when valid[i] = 0.  valid[i] = 1
+ * iff the record parses, d is in range and SM3(x2 || M' || y2) equals C3 (compared without an early exit).  Replaces
+ * DecryptingKey::decrypt / decrypt_digest::<Sm3> (sm2/src/pke/decrypting.rs:174-222). */
+ecg_status ecg_sm2pke_decrypt_batch(ecg_ctx* ctx, size_t n, const uint8_t* cts, const uint64_t* offsets, const uint8_t* d32,
+                                    int mode, uint8_t* out, uint64_t* pt_len, uint8_t* valid);
 
 /* SEC1 compressed point decoding (rank 2 of SURVEY 8(f)): records of 1 + FB bytes (02|03 || x; all zero bytes = the
  * identity; 33 bytes for the 256-bit curves, 49 for the 384-bit ones, 29 for P-224, 25 for P-192, 67 for P-521).

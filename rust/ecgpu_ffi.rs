@@ -83,6 +83,12 @@ unsafe extern "C" {
                                    low_s_only: i32, out_xy: *mut u8, valid: *mut u8) -> i32;
     /// `sm2::dsa::VerifyingKey::verify_prehash` over a batch (sm2/src/dsa/verifying.rs:138-175)
     pub fn ecg_sm2dsa_verify_batch(ctx: *mut ecg_ctx, n: usize, e32: *const u8, sig64: *const u8, q_xy: *const u8, valid: *mut u8) -> i32;
+    /// `sm2::pke::EncryptingKey::encrypt` over a batch with the caller's ephemeral scalars (sm2/src/pke/encrypting.rs:166-230)
+    pub fn ecg_sm2pke_encrypt_batch(ctx: *mut ecg_ctx, n: usize, msgs: *const u8, offsets: *const u64, k32: *const u8, pb_xy: *const u8,
+                                    mode: i32, compressed: i32, out: *mut u8, status: *mut u8) -> i32;
+    /// `sm2::pke::DecryptingKey::decrypt` over a batch (sm2/src/pke/decrypting.rs:174-222)
+    pub fn ecg_sm2pke_decrypt_batch(ctx: *mut ecg_ctx, n: usize, cts: *const u8, offsets: *const u64, d32: *const u8, mode: i32,
+                                    out: *mut u8, pt_len: *mut u64, valid: *mut u8) -> i32;
     /// `AffinePoint::decompress` over a batch (primeorder/src/affine.rs:179-198)
     pub fn ecg_decompress_batch(ctx: *mut ecg_ctx, curve: i32, n: usize, sec1_33: *const u8, out_xy: *mut u8,
                                 out_inf: *mut u8, valid: *mut u8) -> i32;
@@ -318,6 +324,57 @@ impl GpuEngine {
         // SAFETY: as above.
         let rc = unsafe { ecg_sm2dsa_verify_batch(self.ctx, n, e.as_ptr().cast(), sig.as_ptr().cast(), q_xy.as_ptr().cast(), valid.as_mut_ptr()) };
         self.check(rc).map(|_| valid.into_iter().map(|v| v != 0).collect())
+    }
+
+    /// `EncryptingKey::encrypt` (mode C1C3C2 = 0 / C1C2C3 = 1, digest SM3) over a slice of messages for one recipient key,
+    /// with the caller's ephemeral scalars (the reference draws k from its RNG inside `encrypt`).  `Ok(None)` at i where
+    /// the KDF output was all zero (draw another k and retry that message) or the message / k was refused.
+    pub fn sm2pke_encrypt_batch(&mut self, pb: &PointXY, k: &[Bytes32], msgs: &[&[u8]], mode: i32, compressed: bool)
+                                -> Result<Vec<Option<Vec<u8>>>, GpuError> {
+        let n = msgs.len();
+        assert!(k.len() == n);
+        let ovh = 32 + if compressed { 33 } else { 65 };
+        let mut offsets = Vec::with_capacity(n + 1);
+        let mut data = Vec::new();
+        offsets.push(0u64);
+        for m in msgs {
+            data.extend_from_slice(m);
+            offsets.push(data.len() as u64);
+        }
+        let pbs: Vec<PointXY> = vec![*pb; n];
+        let (mut out, mut status) = (vec![0u8; data.len() + n * ovh], vec![0u8; n]);
+        // SAFETY: `data` holds offsets[n] bytes, `offsets` n + 1 values, `k` / `pbs` n records, `out` offsets[n] + n * ovh bytes.
+        let rc = unsafe {
+            ecg_sm2pke_encrypt_batch(self.ctx, n, data.as_ptr(), offsets.as_ptr(), k.as_ptr().cast(), pbs.as_ptr().cast(), mode,
+                                     compressed as i32, out.as_mut_ptr(), status.as_mut_ptr())
+        };
+        self.check(rc).map(|_| (0..n).map(|i| {
+            let (lo, hi) = (offsets[i] as usize + i * ovh, offsets[i + 1] as usize + (i + 1) * ovh);
+            if status[i] == 1 { Some(out[lo..hi].to_vec()) } else { None }
+        }).collect())
+    }
+
+    /// `DecryptingKey::decrypt` over a slice of ciphertexts under one secret key: `None` where the reference returns `Err`.
+    pub fn sm2pke_decrypt_batch(&mut self, d: &Bytes32, cts: &[&[u8]], mode: i32) -> Result<Vec<Option<Vec<u8>>>, GpuError> {
+        let n = cts.len();
+        let mut offsets = Vec::with_capacity(n + 1);
+        let mut data = Vec::new();
+        offsets.push(0u64);
+        for c in cts {
+            data.extend_from_slice(c);
+            offsets.push(data.len() as u64);
+        }
+        let ds: Vec<Bytes32> = vec![*d; n];
+        let (mut out, mut len, mut valid) = (vec![0u8; data.len()], vec![0u64; n], vec![0u8; n]);
+        // SAFETY: `data` / `out` hold offsets[n] bytes, `offsets` n + 1 values, `ds` / `len` / `valid` n records.
+        let rc = unsafe {
+            ecg_sm2pke_decrypt_batch(self.ctx, n, data.as_ptr(), offsets.as_ptr(), ds.as_ptr().cast(), mode, out.as_mut_ptr(), len.as_mut_ptr(),
+                                     valid.as_mut_ptr())
+        };
+        self.check(rc).map(|_| (0..n).map(|i| {
+            let lo = offsets[i] as usize;
+            if valid[i] != 0 { Some(out[lo..lo + len[i] as usize].to_vec()) } else { None }
+        }).collect())
     }
 
     /// `AffinePoint::decompress` over a batch of SEC1 compressed records: `None` where decoding fails.

@@ -7,7 +7,7 @@ import os, random, sys
 import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path[:0] = [os.path.join(ROOT, "elliptic-curves_b200"), os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tests")]
-import ecgpu, pyref, ecref
+import ecgpu, pyref, ecref, sm2pke_ref
 from helpers import pack_scalars, pack_points, unpack_points
 
 def main():
@@ -66,6 +66,19 @@ def main():
         pk[i] = np.frombuffer(px, np.uint8); sg[i] = np.frombuffer(s64, np.uint8)
         assert pyref.bip340_verify(px, msg[i].tobytes(), s64)
     assert eng.schnorr_verify_batch(pk, msg, sg).all()
+    # SM2 public-key encryption: both entries, both layouts, both C1 forms, a refused record (empty message)
+    c = pyref.CURVES["sm2"]
+    d = rng.randrange(1, c.n); Pb = pyref.mul(c, d, pyref.G(c))
+    pb = Pb[0].to_bytes(32, "big") + Pb[1].to_bytes(32, "big")
+    msgs = [os.urandom(L) for L in (0, 1, 31, 32, 33, 56, 64, 65, 200, 1000)]
+    kk = [rng.randrange(1, c.n) for _ in msgs]
+    K = np.frombuffer(b"".join(k.to_bytes(32, "big") for k in kk), np.uint8)
+    for mode in (0, 1):
+        for compressed in (True, False):
+            cts, st = eng.sm2pke_encrypt_vartime(msgs, K, pb, mode, compressed)
+            assert st.tolist() == [0] + [1] * 9, ("sm2pke", st)
+            assert cts[3] == sm2pke_ref.sm2pke_encrypt(Pb, kk[3], msgs[3], mode, compressed)[1], ("sm2pke", "encrypt")
+            assert eng.sm2pke_decrypt_vartime([x or b"" for x in cts], d.to_bytes(32, "big"), mode) == [None] + msgs[1:], ("sm2pke", "decrypt")
     eng.close()
     print("sanitize workload OK")
 
